@@ -18,6 +18,10 @@ prints ONE JSON line on rank 0.
             Weights (7.2 GB) are >> L2 (126 MB), so every launch streams from HBM.
   cpu_baseline  the CPU oracle (port of the reference CUDA forward) on the host cores, a few
             tokens of the same model.
+  --dump-outputs DIR   after the timed decode, what its last step computed, as a caller of the engine receives it:
+            DIR/logits.npy (f32 [50277]) and DIR/state_{xy,aa,bb,pp,dd}.npy (f64 [L*E], the recurrent state the
+            next token continues from; rank 0's copy when N > 1). The model and the token are seeded, so two
+            builds run with the same arguments can be compared array by array.
   --impl reference   the UNMODIFIED reference CUDA build (oracle/_ref/ref_harness, compiled from
             /root/reference by oracle/Makefile) on GPU 0, same .bin, greedy decode through its
             own RWKV::forward, wall clock — the reference has no CPU forward (SURVEY.md 8c);
@@ -35,6 +39,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark runs from the tree build() left and writes nothing into it
 
 SHAPES = {"169m": (12, 768), "1b5": (24, 2048), "7b": (32, 4096), "14b": (40, 5120)}
 SEED = 20240924
@@ -196,6 +201,15 @@ def ncu_traffic(kernel, workload):
     return None
 
 
+def dump_outputs(out_dir, eng):
+    """The last step's logits and the state after it, read back from the device after the timed region."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "logits.npy"), eng.debug_read("logits"))
+    for k, v in eng.state_download().items():
+        np.save(os.path.join(out_dir, "state_%s.npy" % k), v)
+
+
 _REAL_STDOUT = None
 
 
@@ -227,6 +241,8 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=None, choices=sorted(SHAPES))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the logits and the recurrent state of the last timed step as DIR/<name>.npy")
     ap.add_argument("--parallelism", default="tp", choices=["tp", "replicas"],
                     help="N > 1: which arrangement the headline `value` reports. 'tp' (default) = ONE stream decoded by the "
                          "N GPUs together (strong scaling: column/row split of every matrix, two in-kernel NVLink exchanges "
@@ -241,7 +257,6 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     workload = args.workload or "7b"
     pkg = importlib.import_module("rwkv-cpp-accelerated_b200")
-    pkg.build.build_all(force=False)
 
     if args.impl == "reference":
         run_reference(args, pkg, workload)
@@ -292,6 +307,8 @@ def main():
     ms = eng.decode_timed([SEED_TOKEN] * args.steps, teacher_forced=False)
     sync_all()
     launches = eng.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng)
     t = torch.tensor([ms], dtype=torch.float64, device="cuda:%d" % local_rank)
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -112,8 +112,10 @@ def file_bytes(L, E, V=50277):
 
 
 def genmodel(n_layers, n_embed, seed, path, threads=None):
-    """Write a synthetic reference-format model file (see tools/genmodel.cpp)."""
-    build_genmodel()
+    """Write a synthetic reference-format model file (see tools/genmodel.cpp). Uses the generator build() made, so
+    that bench.py can make its model from a read-only tree; builds it only when it is missing."""
+    if not os.path.exists(GENMODEL):
+        build_genmodel()
     cmd = [GENMODEL, str(n_layers), str(n_embed), str(seed), path]
     if threads:
         cmd.append(str(threads))

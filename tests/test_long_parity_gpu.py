@@ -1,78 +1,53 @@
 """Parity at the sizes and lengths BASELINE.json names, against the REFERENCE ITSELF (the unmodified
-rwkv.cu + rwkv.h built into oracle/_ref/ref_harness, run on this GPU): the reference decodes greedily,
-the engine replays the same tokens teacher-forced, logits are compared step by step and the recurrent
-state at the end. Plus two stress models for the fixed-point activation quantiser and the layernorm
-statistics: outlier channels and a tiny residual stream.
+rwkv.cu + rwkv.h, run on a B200; its runs are stored under tests/golden/reference/ by
+tests/golden/make_reference_golden.py): the reference decodes greedily, the engine replays the same tokens
+teacher-forced, logits are compared step by step and the recurrent state at the end. Plus stress models for the
+fixed-point activation quantiser and the layernorm statistics: outlier channels and a tiny or offset residual stream.
 
 Tolerance (north_star): logits within 1e-3 of max|logits|; arg-max identical wherever the reference's own
-top-1 / top-2 margin exceeds 1e-3 of max|logits|."""
-import os
-import shutil
-import subprocess
+top-1 / top-2 margin exceeds 1e-3 of max|logits|. A stored run keeps a sample of each logit vector and of the
+state (tests/util.py:shrink_reference_run); the tolerance applies to every stored entry."""
 import sys
 
 import numpy as np
 import pytest
 
-from util import ROOT
+from util import (ROOT, STATE_KEYS, load_reference, reference_logits_err, reference_margin, reference_state_err,
+                  stress_model)
 
 pytestmark = pytest.mark.gpu
 
 REL_TOL = 1e-3
 SEED_TOKEN = 4118
-VOCAB = 50277
 
 
 def rel_err(got, ref):
     return float(np.abs(got.astype(np.float64) - ref.astype(np.float64)).max() / max(np.abs(ref).max(), 1e-6))
 
 
-def margin(ref):
-    top = np.partition(ref, -2)[-2:]
-    return float((top.max() - top.min()) / max(np.abs(ref).max(), 1e-6))
-
-
-def reference_run(path, n_tokens, dump_every, tmp_path, tokens=None):
-    """Greedy decode of `n_tokens` by the reference binary (or teacher-forced on `tokens`)."""
-    from oracle.oracle import REF_HARNESS, read_ref_dump
-    if not os.path.exists(REF_HARNESS):
-        pytest.skip("oracle/_ref/ref_harness not built (needs /root/reference at build time)")
-    tf = tmp_path / "seed.txt"
-    tf.write_text("\n".join(map(str, tokens)) if tokens else "%d\n" % SEED_TOKEN)
-    dump = tmp_path / "ref.bin"
-    cmd = [REF_HARNESS, path, str(tf), str(dump), "--dump-every", str(dump_every)]
-    if not tokens:
-        cmd += ["--greedy", str(n_tokens)]
-    r = subprocess.run(cmd, capture_output=True, text=True, timeout=1200)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    d = read_ref_dump(str(dump))
-    toks = [int(x) for x in open(str(dump) + ".tokens").read().split()]
-    os.remove(str(dump))
-    return d, toks
-
-
-def compare_with_reference(pkg, path, n_tokens, dump_every, tmp_path, tokens=None):
-    d, toks = reference_run(path, n_tokens, dump_every, tmp_path, tokens)
+def compare_with_reference(pkg, path, case, n_tokens, dump_every=1):
+    ref = load_reference(case)
+    toks = [int(t) for t in ref["tokens"]]
     assert len(toks) >= n_tokens
-    want = dict(zip(d["steps"], d["logits"]))
+    want = {int(s): i for i, s in enumerate(ref["steps"])}
+    assert all(s in want for s in range(0, n_tokens, dump_every))
     eng = pkg.Engine(path)
     worst, checked = 0.0, 0
     for step in range(n_tokens):
         if step in want:
+            i = want[step]
             got = eng.forward([toks[step]])[0]
-            ref = want[step]
-            e = rel_err(got, ref)
+            e = reference_logits_err(got, ref, i)
             worst = max(worst, e)
             assert e < REL_TOL, "step %d: logits rel err %.3g" % (step, e)
-            if margin(ref) > 1e-3:
-                assert int(got.argmax()) == int(ref.argmax()), "step %d argmax" % step
+            if reference_margin(ref, i) > 1e-3:
+                assert int(got.argmax()) == int(ref["argmax"][i]), "step %d argmax" % step
                 checked += 1
         else:
             eng.forward([toks[step]], want_logits=False)
     st = eng.state_download()
-    for k in ("xy", "aa", "bb", "dd"):
-        ref = d["state"][k]
-        assert np.abs(st[k] - ref).max() / max(np.abs(ref).max(), 1e-6) < REL_TOL, "state %s" % k
+    for k in STATE_KEYS:
+        assert reference_state_err(st[k], ref, k) < REL_TOL, "state %s" % k
     eng.close()
     return worst, checked, len(want)
 
@@ -89,35 +64,10 @@ def bench_model(pkg, workload):
     ("7b", 64, 1),       # BASELINE config 4 (headline): the bench model itself
     ("14b", 64, 1),      # BASELINE config 5 at full depth (40 x 5120) on one GPU
 ])
-def test_decode_matches_the_reference_at_baseline_sizes(pkg, tmp_path, workload, n_tokens, dump_every):
-    worst, checked, compared = compare_with_reference(pkg, bench_model(pkg, workload), n_tokens, dump_every, tmp_path)
+def test_decode_matches_the_reference_at_baseline_sizes(pkg, workload, n_tokens, dump_every):
+    worst, checked, compared = compare_with_reference(pkg, bench_model(pkg, workload), workload, n_tokens, dump_every)
     print("%s x %d tokens vs the reference CUDA build: worst logits rel err %.3g over %d compared steps, argmax checked on %d"
           % (workload, n_tokens, worst, compared, checked))
-
-
-def _stress_model(make_model, tmp_path, kind):
-    """A copy of the 3 x 768 synthetic model with its layernorm parameters edited in place.
-    LAYERNORMS = f64 [4(L+1)][E] after xbuf (f64 [E]) and embed (f32 [V][E]): rows 0,1 = ln0 w,b;
-    4i+2, 4i+3 = ln1 of layer i; 4(i+1), 4(i+1)+1 = ln2 of layer i (convert_model.py:30-46)."""
-    L, E = 3, 768
-    src = make_model(L, E)
-    dst = str(tmp_path / ("stress_%s.bin" % kind))
-    shutil.copyfile(src, dst)
-    ln = np.memmap(dst, dtype=np.float64, mode="r+", offset=16 + 8 * E + 4 * VOCAB * E, shape=(4 * (L + 1), E))
-    if kind == "outliers":
-        rng = np.random.default_rng(7)
-        for i in range(L):
-            ch = rng.choice(E, size=3, replace=False)
-            ln[4 * i + 2, ch] *= 300.0      # ln1 weight: three channels 300x the rest
-            ln[4 * (i + 1), ch] *= 300.0    # ln2 weight
-    elif kind == "tiny_residual":
-        ln[0] *= 1e-3                       # ln0 weight and bias: residual stream of magnitude 1e-3
-        ln[1] *= 1e-3
-    elif kind == "offset_residual":
-        ln[1] += 50.0                       # ln0 bias: |mean| >> std in every later layernorm
-    ln.flush()
-    del ln
-    return dst
 
 
 @pytest.mark.parametrize("kind", ["outliers", "tiny_residual", "offset_residual"])
@@ -126,7 +76,7 @@ def test_stress_models_match_oracle_and_reference(pkg, make_model, tmp_path, kin
     the typical element few quantisation levels of the per-vector scale; a residual stream of magnitude 1e-3 or
     with |mean| >> std probes the layernorm statistics."""
     from oracle.oracle import Oracle
-    path = _stress_model(make_model, tmp_path, kind)
+    path = stress_model(make_model(3, 768), str(tmp_path / ("stress_%s.bin" % kind)), kind)
     orc = Oracle(path)
     eng = pkg.Engine(path)
     toks, tok, worst = [], SEED_TOKEN, 0.0
@@ -141,5 +91,5 @@ def test_stress_models_match_oracle_and_reference(pkg, make_model, tmp_path, kin
         tok = int(ref.argmax())
     eng.close()
     orc.close()
-    w2, _, _ = compare_with_reference(pkg, path, 8, 1, tmp_path, tokens=toks)
+    w2, _, _ = compare_with_reference(pkg, path, kind, 8)
     print("%s: worst logits rel err vs oracle %.3g, vs the reference CUDA build %.3g" % (kind, worst, w2))

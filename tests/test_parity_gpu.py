@@ -1,15 +1,14 @@
-"""GPU parity: the CUDA engine (through the C ABI) vs the CPU oracle, and the oracle vs the
-unmodified reference CUDA build (oracle/_ref/ref_harness) where that binary exists.
+"""GPU parity: the CUDA engine (through the C ABI) vs the CPU oracle, and the oracle vs a stored run of the
+unmodified reference CUDA build (tests/golden/reference/).
 
 Tolerance (BASELINE.json north_star): logits within 1e-3 relative to the vector's
 max-abs; argmax identical wherever the reference's own top-1/top-2 margin exceeds 1e-3
 of max-abs (SURVEY.md H5: below that the reference's fp32 atomics decide the winner).
 """
-import os
-import subprocess
-
 import numpy as np
 import pytest
+
+from util import STATE_KEYS, load_reference, reference_logits_err, reference_margin, reference_state_err
 
 pytestmark = pytest.mark.gpu
 
@@ -204,42 +203,30 @@ def test_errors(pkg, make_model, tmp_path):
     e.close()
 
 
-def test_oracle_vs_reference_cuda(pkg, make_model, tmp_path):
-    """Pins the oracle: the UNMODIFIED reference (rwkv.cu + rwkv.h, built by oracle/Makefile
-    into oracle/_ref/) runs on this GPU on the same .bin and token stream."""
-    from oracle.oracle import Oracle, REF_HARNESS, read_ref_dump
-    if not os.path.exists(REF_HARNESS):
-        pytest.skip("oracle/_ref/ref_harness not built (needs /root/reference at build time)")
+def test_oracle_vs_reference_cuda(pkg, make_model):
+    """Pins the oracle: the UNMODIFIED reference (rwkv.cu + rwkv.h) run on a B200 on the same .bin and token
+    stream, stored as tests/golden/reference/oracle_3x768.npz by tests/golden/make_reference_golden.py."""
+    from oracle.oracle import Oracle
+    ref = load_reference("oracle_3x768")
+    assert ref["steps"].tolist() == list(range(8))
+    toks = [int(t) for t in ref["tokens"]]
     path = make_model(3, 768)
     orc = Oracle(path)
-    toks, tok, ref_logits = [], SEED_TOKEN, []
-    for _ in range(8):
-        toks.append(tok)
-        lg = orc.forward(tok)
-        ref_logits.append(lg)
-        tok = int(lg.argmax())
-    tf = tmp_path / "toks.txt"
-    tf.write_text("\n".join(map(str, toks)))
-    dump = tmp_path / "ref.bin"
-    r = subprocess.run([REF_HARNESS, path, str(tf), str(dump)], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    d = read_ref_dump(str(dump))
-    assert d["steps"] == list(range(8))
     worst = 0.0
-    for got, ref in zip(ref_logits, d["logits"]):
-        worst = max(worst, rel_err(got, ref))
+    for i, t in enumerate(toks):
+        worst = max(worst, reference_logits_err(orc.forward(t), ref, i))
     print("oracle vs reference CUDA: worst logits rel err %.3g" % worst)
     assert worst < 1e-4
-    for k in ("xy", "aa", "bb", "dd"):
-        ref = d["state"][k]
-        assert np.abs(orc.state[k] - ref).max() / max(np.abs(ref).max(), 1e-6) < 1e-4, k
+    for k in STATE_KEYS:
+        assert reference_state_err(orc.state[k], ref, k) < 1e-4, k
+    orc.close()
     # and the engine against the reference itself, same stream
     eng = pkg.Engine(path)
-    for t, ref in zip(toks, d["logits"]):
+    for i, t in enumerate(toks):
         got = eng.forward([t])[0]
-        assert rel_err(got, ref) < REL_TOL
-        if margin(ref) > 1e-3:
-            assert int(got.argmax()) == int(ref.argmax())
+        assert reference_logits_err(got, ref, i) < REL_TOL
+        if reference_margin(ref, i) > 1e-3:
+            assert int(got.argmax()) == int(ref["argmax"][i])
     eng.close()
 
 
