@@ -324,6 +324,28 @@ class RWKV {
         return typical_with_u(out, temp, u);
     }
 
+    // Extension: free-running generation on the device (rwkv_b200_generate). Same tokens, same state and same
+    // position of the process-wide generator as the loop `forward(token); token = sample(temp);` run n times, or
+    // until it produces one of the `stop` ids - without a host round trip per token. Returns t1..tk; the state has
+    // consumed token, t1, ..., t(k-1) and `out` holds the logits of the last forward.
+    std::vector<unsigned long long> generate(unsigned long long token, unsigned long long n, float temp = 0.9f,
+                                             std::vector<unsigned long long> stop = {}) {
+        // The loop's uniforms, drawn from a copy of the generator; the generator itself advances by the steps that
+        // ran (generate_canonical<double, 53> on mt19937_64 takes exactly one draw).
+        std::mt19937_64 gen = rwkv_sampler_generator();
+        std::vector<double> u(n);
+        for (double &x : u) x = std::generate_canonical<double, 53>(gen);
+        std::vector<unsigned long long> toks = runGenerate(token, n, RWKV_B200_GEN_TYPICAL, temp, u.data(), stop);
+        rwkv_sampler_generator().discard(toks.size());
+        return toks;
+    }
+
+    // Extension: the same for the greedy loop `forward(token); token = argmax(out);`.
+    std::vector<unsigned long long> generateGreedy(unsigned long long token, unsigned long long n,
+                                                   std::vector<unsigned long long> stop = {}) {
+        return runGenerate(token, n, RWKV_B200_GEN_GREEDY, 1.0f, nullptr, stop);
+    }
+
     RWKVState emptyState() { return {num_layers, num_embed, 1}; }
 
     long long loadContext(std::string input, bool progress = false) {
@@ -351,6 +373,28 @@ class RWKV {
         }
         delete[] tensors;
         delete tokenizer;
+    }
+
+  private:
+    std::vector<unsigned long long> runGenerate(unsigned long long token, unsigned long long n, int how, float temp,
+                                                const double *uniforms, const std::vector<unsigned long long> &stop) {
+        if (!ready) throw std::runtime_error("RWKV not loaded");
+        if (n == 0) return {};
+        if (strictState || state->hostAhead) { // as in forward: one token on slot 0
+            const unsigned long long slots = strictState ? 1ull : state->stateSize;
+            if (rwkv_b200_state_upload(engine, state->statexy, state->stateaa, state->statebb, nullptr, state->statedd,
+                                       std::min(slots, state->stateSize)) != 0)
+                throw std::runtime_error(std::string("RWKV state upload failed: ") + rwkv_b200_last_error());
+            state->hostAhead = false;
+        }
+        std::vector<unsigned long long> toks(n);
+        unsigned long long k = 0;
+        if (rwkv_b200_generate(engine, token, n, how, temp, uniforms, stop.data(), (int)stop.size(), toks.data(), &k, out) != 0)
+            throw std::runtime_error(std::string("RWKV generate failed: ") + rwkv_b200_last_error());
+        state->deviceAhead = true;
+        if (strictState) state->syncToHost();
+        toks.resize(k);
+        return toks;
     }
 };
 

@@ -169,12 +169,44 @@ unsigned long long rwkv_b200_launch_count(const rwkv_b200_model *m);
 int rwkv_b200_sample_typical(rwkv_b200_model *m, float temp, double u, unsigned long long *token,
                              double *margin);
 
+/* Free-running generation on state slot 0: exactly `n` iterations of
+ *     logits = forward(tok); tok = pick(logits)
+ * starting from `first_token`, as back-to-back launches of the token kernel that pick the
+ * next token on the device (no host round trip per token). pick is
+ *   RWKV_B200_GEN_GREEDY : the arg-max (first index of the largest logit);
+ *   RWKV_B200_GEN_TYPICAL: typical_with_u(logits, temp, uniforms[i]) of
+ *                          include/rwkv/sampler/typical.h, i.e. exactly what
+ *                          rwkv_sampler_pick returns on the host for that uniform. The device
+ *                          sums differ from the host's sequential ones by ~1e-13, so a step
+ *                          whose uniform lies closer than set_option "sample_margin" (default
+ *                          1e-9) to an interval boundary is finished on the host with the same
+ *                          uniform: the result is always the host sampler's token stream.
+ * `uniforms`: n values in [0, 1) (TYPICAL only; may be NULL for GREEDY), one per step, e.g.
+ * std::generate_canonical<double, 53> draws of the caller's generator. `temp` > 1/256.
+ * `stop`: up to 8 token ids; the run ends after the first step that produces one of them.
+ * After the call the state has consumed first_token, t1, ..., t(k-1); tokens_out[0..k) =
+ * t1..tk with k = *n_out, and k < n only if tk is a stop id. The device logits, and
+ * `logits_out` (50277 floats) if not NULL, are those of the last forward, so
+ * rwkv_b200_sample_typical and rwkv_b200_logits_host stay consistent with it.
+ * Errors (no device work done): tensor parallelism (tp_size > 1 is not supported), a token
+ * or stop id >= vocabulary, a uniform outside [0, 1), n == 0, a NULL output.
+ * No reference counterpart (the reference samples on the host after every forward). */
+#define RWKV_B200_GEN_GREEDY 0
+#define RWKV_B200_GEN_TYPICAL 1
+int rwkv_b200_generate(rwkv_b200_model *m, unsigned long long first_token, unsigned long long n,
+                       int how, float temp, const double *uniforms,
+                       const unsigned long long *stop, int n_stop,
+                       unsigned long long *tokens_out, unsigned long long *n_out,
+                       float *logits_out);
+
 /* Engine knobs (all optional), key/value strings: "window" / "bwindow" (bulk copies in
  * flight per SM while streaming / while the CTAs exchange vectors), "pf_dist" (tiles the L2
  * prefetch runs ahead), "stages" (ring depth), "poll_first", "timeout_ms", "max_layers",
  * "trace", "prefill", "prefill_min", "prefill_graph", "grid" (CTAs, at most the SM count),
  * "cluster" (1, 2 or 4 CTAs share a gather through distributed shared memory; measured
- * without gain, default 1). Returns non-zero for an unknown key. */
+ * without gain, default 1), "sample_margin" (rwkv_b200_generate: smallest distance of a
+ * uniform to an interval boundary the device's sampled token is kept at, in [0, 1], default
+ * 1e-9). Returns non-zero for an unknown key. */
 int rwkv_b200_set_option(rwkv_b200_model *m, const char *key, const char *value);
 
 /* --- tensor-parallel wiring (tp_size > 1 only) --------------------------------- */

@@ -41,6 +41,11 @@ class ModelWrapper:
         CPP_LIB.modelForward(self.cpp_instance, token)
         return (self.get_output(), self.get_state())
 
+    def generate(self, token: int, n: int, temp: float = 0.9, stop: Iterable[int] = (), greedy: bool = False):
+        """Up to n tokens generated on the device from `token`: the tokens `forward` + `sample(temp)` (or + arg-max
+        with greedy=True) in a loop would give, ending early after a token in `stop`."""
+        return CPP_LIB.generate(self.cpp_instance, token, n, temp, list(stop), greedy)
+
 
 class TokenizerWrapper:
 

@@ -80,6 +80,17 @@ static int typicalSample(void *h, float temp = 0.9, float tau = 0.8) {
     return static_cast<RWKV *>(h)->sample(temp, tau);
 }
 
+// Not in the reference binding: RWKV::generate / generateGreedy (free-running generation on the device), the same
+// tokens as modelForward + typicalSample (or + arg-max) in a loop.
+static std::vector<unsigned long long> generate(void *h, int64_t token, int64_t n, float temp, std::vector<unsigned long long> stop,
+                                                bool greedy) {
+    if (token < 0 || n < 0) throw py::value_error("generate: token and n must be non-negative");
+    RWKV *net = static_cast<RWKV *>(h);
+    py::gil_scoped_release release;
+    return greedy ? net->generateGreedy((unsigned long long)token, (unsigned long long)n, stop)
+                  : net->generate((unsigned long long)token, (unsigned long long)n, temp, stop);
+}
+
 static std::tuple<int64_t, int64_t> loadWrapper(void *h, const std::string &filename) {
     RWKV *net = static_cast<RWKV *>(h);
     net->loadFile(filename);
@@ -108,4 +119,6 @@ PYBIND11_MODULE(rwkv, m) {
     m.def("tokenizerDecode", &tokenizerDecode, "tokenizerDecode");
 
     m.def("typicalSample", &typicalSample, "typicalSample", py::arg("handle"), py::arg("temp") = 0.9f, py::arg("tau") = 0.8f);
+    m.def("generate", &generate, "generate", py::arg("handle"), py::arg("token"), py::arg("n"), py::arg("temp") = 0.9f,
+          py::arg("stop") = std::vector<unsigned long long>{}, py::arg("greedy") = false);
 }

@@ -1,7 +1,7 @@
 """In-tree builds (no JIT cache): every artefact lands next to its sources so that it
 travels to the GPU box with the repo snapshot.
 
-  librwkv_b200.so        csrc/engine.cu + kernels.cuh      nvcc, sm_100a only
+  librwkv_b200.so        csrc/engine.cu + generate_kernels.cu + kernels.cuh   nvcc, sm_100a only
   tools/genmodel         tools/genmodel.cpp                g++
   bindings/pybind/rwkv*.so   bindings/pybind/c_binding.cpp g++ + pybind11, links librwkv_b200.so
   oracle/librwkv_oracle.so, oracle/_ref/*                  oracle/Makefile (checker only)
@@ -52,9 +52,10 @@ def nvcc():
 def build_engine(force=False):
     srcs = [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC))]
     srcs.append(os.path.join(ROOT, "include", "rwkv_b200.h"))
+    srcs.append(os.path.join(ROOT, "include", "rwkv", "sampler", "typical.h"))
     if force or _newer(LIB, srcs):
         tmp = LIB + ".tmp%d" % os.getpid()  # a snapshot taken during the build never sees a half-written library
-        _run([nvcc()] + NVCC_FLAGS + ["-o", tmp, os.path.join(CSRC, "engine.cu")])
+        _run([nvcc()] + NVCC_FLAGS + ["-o", tmp, os.path.join(CSRC, "engine.cu"), os.path.join(CSRC, "generate_kernels.cu")])
         os.replace(tmp, LIB)
     return LIB
 

@@ -35,13 +35,15 @@ constexpr int kTraceMax = 2048;            // trace stamps per CTA (debug)
 constexpr int kTileTraceMax = 4096;        // tiles per CTA recorded by the tile trace (debug)
 constexpr int kQMax = 4194303;             // 2^22 - 1: largest |q| of the activation quantiser
 constexpr int kSmemLimit = 232448;         // opt-in dynamic shared memory per CTA on sm_100
+constexpr int kMaxStop = 8;                // stop ids of a generate run
 
 // Device-resident control block of one model (one per rank).
 struct Ctrl {
     unsigned long long token; // input token of the current forward (feed_mode 0)
     unsigned long long next;  // argmax of the last logits (greedy)
     unsigned long long slot;  // state slot (PARRALEL mode)
-    unsigned long long pos;   // cursor into a device-resident token stream (feed_mode 2)
+    unsigned long long pos;   // cursor into a device-resident token stream (feed_mode 2); generate: steps done
+    unsigned long long halt;  // generate: nonzero = the next launches exit at entry (stop token or small margin)
 };
 
 // Diagnostic record written to mapped host memory just before a timeout trap, so that the host can say
@@ -53,7 +55,8 @@ struct Diag {
     unsigned long long aux;
 };
 constexpr unsigned int kDiagStats = 1, kDiagVec = 2, kDiagOff = 3, kDiagPeerSum = 4, kDiagSr = 5, kDiagDone = 6,
-                       kDiagArg = 7, kDiagRingFull = 8, kDiagRingEmpty = 9, kDiagPlanesFree = 10, kDiagPlanesReady = 11;
+                       kDiagArg = 7, kDiagRingFull = 8, kDiagRingEmpty = 9, kDiagPlanesFree = 10, kDiagPlanesReady = 11,
+                       kDiagSample = 12;
 
 // Everything the token kernel needs, passed by value (__grid_constant__).
 // G ranks (GPUs) decode ONE stream together (G = 1: a single GPU). Split (SURVEY 8e):
@@ -120,6 +123,16 @@ struct Params {
     unsigned long long off_saa, off_sbb; // [slots][L][E] f64 WKV state (every rank holds all channels)
     unsigned long long *trace;  // optional [grid][kTraceMax] globaltimer stamps (debug), or nullptr
     unsigned long long *ptrace; // optional [2][grid][kTileTraceMax]: tile issue / tile ready times (debug)
+    // ---- generate launches only (k_token<.., GEN = true>; greedy = 1: arg-max, 0: typical sampler) ----
+    // (kept behind every other field: the offsets the other instantiations read do not move)
+    unsigned int off_smp;       // [kRep][3][grid] tagged doubles: per-CTA sampler partials (max, sum exp, sum exp^e)
+    int exponent;               // uint8(1 / temp) of the reference sampler: 0 = uniform draw
+    int n_stop;                 // stop ids in `stop`
+    double margin_min;          // a sampled token whose uniform lies closer than this to a boundary halts the run
+    const double *uniforms;     // [n] the uniforms of the run, indexed by ctrl->pos
+    unsigned long long *gen_tokens; // [n] token of step ctrl->pos
+    double *gen_margins;        // [n] its margin (typical)
+    unsigned long long stop[kMaxStop];
 };
 
 // ---------------------------------------------------------------------------------------

@@ -27,11 +27,16 @@
 #include <cuda_runtime.h>
 
 #include "../../include/rwkv/enums/enum.h"
+#include "../../include/rwkv/sampler/typical.h"
 #include "../../include/rwkv_b200.h"
 #include "aux_kernels.cuh"
 #include "binfmt.h"
 #include "prefill.cuh"
 #include "token_kernel.cuh"
+
+namespace rk {
+const void *token_entry_gen(int cpl, bool full); // generate_kernels.cu
+}
 
 namespace {
 
@@ -65,6 +70,10 @@ struct rwkv_b200_model {
     int grid = 0;
     int cpl = 0;
     double *d_sample = nullptr, *h_sample = nullptr; // device sampler result {token, margin}
+    // generate: device [cap] uniforms + [cap] tokens + [cap] margins, and a pinned host mirror of the same layout
+    unsigned char *d_gen = nullptr, *h_gen = nullptr;
+    unsigned long long gen_cap = 0;
+    double sample_margin = 1e-9; // set_option "sample_margin": the device's sampled token is kept at or above it
     size_t xch_bytes = 0;   // exchange block (peer-visible with tensor parallelism)
     bool tp_wired = false;  // peers' exchange blocks imported
     std::vector<void *> ipc_opened;
@@ -106,11 +115,11 @@ int sync_failed(M *m, cudaError_t e, const char *what) {
     if (d && d->code) {
         static const char *names[] = {"", "slice statistics", "activation vector", "offset sums", "peer partial sums",
                                       "sigmoid exchange", "completion flags", "arg-max candidates", "ring (full)", "ring (empty)",
-                                      "cluster: limb planes free", "cluster: limb planes written"};
+                                      "cluster: limb planes free", "cluster: limb planes written", "sampler partials"};
         return fail(100 + (int)e,
                     "%s failed: %s; token kernel timed out waiting for %s: rank %u cta %u thread %u layer %u kind %u "
                     "expected tag %u saw %u aux %llu (a peer rank that never launched, or a protocol bug)",
-                    what, cudaGetErrorString(e), d->code < 12 ? names[d->code] : "?", d->rank, d->cta, d->thread, d->layer,
+                    what, cudaGetErrorString(e), d->code < 13 ? names[d->code] : "?", d->rank, d->cta, d->thread, d->layer,
                     d->kind, d->expect, d->seen, d->aux);
     }
     return fail(100 + (int)e, "%s failed: %s", what, cudaGetErrorString(e));
@@ -123,9 +132,9 @@ int sync_failed(M *m, cudaError_t e, const char *what) {
 
 // ---- kernel dispatch on the model width -------------------------------------------------
 // CPL = 16-byte chunks per lane of an n_embed-byte row; FULL = n_embed == CPL * 512 (no tail predicates).
-#define RK_CPLS(X) X(2) X(4) X(6) X(8) X(10)
-
-const void *token_entry(int cpl, bool full, bool trace) {
+// gen: the instantiation of rwkv_b200_generate (no trace stamps; generate_kernels.cu)
+const void *token_entry(int cpl, bool full, bool trace, bool gen = false) {
+    if (gen) return rk::token_entry_gen(cpl, full);
 #define X(A)                                                                                                          \
     if (cpl == A) {                                                                                                   \
         if (trace) return full ? (const void *)rk::k_token<A, true, true> : (const void *)rk::k_token<A, false, true>; \
@@ -166,7 +175,7 @@ void fill_launch(int grid, int cluster, size_t smem, cudaLaunchConfig_t &cfg, cu
     cfg.numAttrs = cluster > 1 ? 2 : 1;
 }
 
-int launch_token(M *m, int feed, bool greedy, const unsigned long long *stream, cudaStream_t s) {
+int launch_token(M *m, int feed, bool greedy, const unsigned long long *stream, cudaStream_t s, bool gen = false) {
     if (m->tp_size > 1 && !m->tp_wired)
         return fail(7, "tensor parallelism: call rwkv_b200_tp_import with every rank's handle before the first forward");
     rk::Params prm = m->p;
@@ -180,7 +189,7 @@ int launch_token(M *m, int feed, bool greedy, const unsigned long long *stream, 
     m->epoch += (unsigned int)prm.L_run + 1u;
     void *args[] = {&prm};
     const bool full = m->E == (unsigned long long)m->cpl * 512ull;
-    const void *fn = token_entry(m->cpl, full, m->p.trace != nullptr);
+    const void *fn = token_entry(m->cpl, full, m->p.trace != nullptr, gen);
     if (!fn) return fail(3, "no kernel for %d chunks per lane", m->cpl);
     // cooperative: all CTAs resident together (they wait for each other's words); clusters of p.cluster CTAs share
     // the gather through distributed shared memory
@@ -378,8 +387,8 @@ int do_load(M *m, const char *path, int quiet) {
     if (p.stages < 2) return fail(5, "n_embed=%llu leaves no room for a two-stage ring", E);
     if (!grid_fits(E, Er, Vr, m->grid)) return fail(5, "a grid of %d CTAs does not fit n_embed=%llu", m->grid, E);
     const bool full = E == (unsigned long long)m->cpl * 512ull;
-    for (int tr = 0; tr < 2; ++tr) {
-        const void *fn = token_entry(m->cpl, full, tr != 0);
+    for (int tr = 0; tr < 3; ++tr) {
+        const void *fn = token_entry(m->cpl, full, tr == 1, tr == 2);
         if (!fn) return fail(3, "no kernel for %d chunks per lane", m->cpl);
         CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, rk::kSmemLimit));
     }
@@ -481,6 +490,7 @@ int do_load(M *m, const char *path, int quiet) {
         p.off_sr = (unsigned int)take(E * 8);
         p.off_arg = (unsigned int)take(G * nb * sizeof(rk::TaggedDouble));
         p.off_done = (unsigned int)take(G * nb * 8);
+        p.off_smp = (unsigned int)take(rk::kRep * 3 * nb * sizeof(rk::TaggedDouble));
         p.off_logits = (unsigned int)take(V * 4);
         p.off_saa = take(sn * 8);
         p.off_sbb = take(sn * 8);
@@ -577,6 +587,8 @@ void rwkv_b200_free(rwkv_b200_model *m) {
     if (m->h_logits) cudaFreeHost(m->h_logits);
     if (m->h_next) cudaFreeHost(m->h_next);
     if (m->h_sample) cudaFreeHost(m->h_sample);
+    if (m->d_gen) cudaFree(m->d_gen);
+    if (m->h_gen) cudaFreeHost(m->h_gen);
     if (m->h_diag) cudaFreeHost(m->h_diag);
     if (m->stream) cudaStreamDestroy(m->stream);
     cudaGetLastError(); // a context killed by a trap makes every call above fail; do not leave that as "last error"
@@ -734,6 +746,112 @@ int rwkv_b200_sample_typical(rwkv_b200_model *m, float temp, double u, unsigned 
     return 0;
 }
 
+int rwkv_b200_generate(rwkv_b200_model *m, unsigned long long first_token, unsigned long long n, int how, float temp,
+                       const double *uniforms, const unsigned long long *stop, int n_stop, unsigned long long *tokens_out,
+                       unsigned long long *n_out, float *logits_out) {
+    int rc = check_model(m);
+    if (rc) return rc;
+    const unsigned long long V = binfmt::kVocab;
+    if (how != RWKV_B200_GEN_GREEDY && how != RWKV_B200_GEN_TYPICAL) return fail(1, "generate: `how` must be GREEDY (0) or TYPICAL (1)");
+    if (n == 0 || !tokens_out || !n_out) return fail(1, "generate: n must be positive and tokens_out, n_out non-null");
+    *n_out = 0;
+    if (m->tp_size > 1) return fail(7, "generate: not supported with tensor parallelism (%d ranks)", m->tp_size);
+    if (first_token >= V) return fail(1, "generate: token id %llu out of range", first_token);
+    if (n_stop < 0 || n_stop > rk::kMaxStop || (n_stop > 0 && !stop)) return fail(1, "generate: 0..%d stop ids", rk::kMaxStop);
+    for (int k = 0; k < n_stop; ++k)
+        if (stop[k] >= V) return fail(1, "generate: stop id %llu out of range", stop[k]);
+    const bool typ = how == RWKV_B200_GEN_TYPICAL;
+    int exponent = 1;
+    if (typ) {
+        if (!uniforms) return fail(1, "generate: TYPICAL needs n uniforms");
+        for (unsigned long long i = 0; i < n; ++i)
+            if (!(uniforms[i] >= 0.0 && uniforms[i] < 1.0)) return fail(1, "generate: uniform %llu = %.17g is outside [0, 1)", i, uniforms[i]);
+        // uint8(1 / temp) as include/rwkv/sampler/typical.h computes it; defined for 1 / temp < 256
+        if (!(temp > 1.0f / 256.0f)) return fail(1, "generate: temp must be > 1/256 (got %g)", (double)temp);
+        exponent = temp != 1.0f ? (int)(uint8_t)(1.0 / (double)temp) : 1;
+    }
+    CK(cudaSetDevice(m->device));
+    if (m->gen_cap < n) {
+        if (m->d_gen) cudaFree(m->d_gen);
+        if (m->h_gen) cudaFreeHost(m->h_gen);
+        m->d_gen = m->h_gen = nullptr;
+        m->gen_cap = 0;
+        CK(cudaMalloc((void **)&m->d_gen, 24 * n));
+        CK(cudaMallocHost((void **)&m->h_gen, 24 * n));
+        m->gen_cap = n;
+    }
+    const unsigned long long cap = m->gen_cap;
+    double *d_u = reinterpret_cast<double *>(m->d_gen), *h_u = reinterpret_cast<double *>(m->h_gen);
+    unsigned long long *d_t = reinterpret_cast<unsigned long long *>(m->d_gen + 8 * cap), *h_t = reinterpret_cast<unsigned long long *>(m->h_gen + 8 * cap);
+    double *d_mg = reinterpret_cast<double *>(m->d_gen + 16 * cap), *h_mg = reinterpret_cast<double *>(m->h_gen + 16 * cap);
+    if (typ) {
+        memcpy(h_u, uniforms, n * sizeof(double));
+        CK(cudaMemcpyAsync(d_u, h_u, n * sizeof(double), cudaMemcpyHostToDevice, m->stream));
+    }
+    rk::Params &p = m->p;
+    p.exponent = exponent;
+    p.n_stop = n_stop;
+    for (int k = 0; k < rk::kMaxStop; ++k) p.stop[k] = k < n_stop ? stop[k] : 0;
+    p.margin_min = m->sample_margin;
+    p.uniforms = d_u;
+    p.gen_tokens = d_t;
+    p.gen_margins = d_mg;
+    auto is_stop = [&](unsigned long long t) { return std::find(stop, stop + n_stop, t) != stop + n_stop; };
+    // exchange epochs after each enqueued launch: launches that exited at entry must not keep theirs (DESIGN 4.1)
+    std::vector<std::pair<unsigned int, unsigned int>> ep(n + 1);
+    std::vector<float> fallback_logits;
+    unsigned long long done = 0, tok = first_token;
+    // The first segment enqueues every step (no halt: one synchronisation per call). After a halt the launches behind
+    // it exited at entry; the next segment enqueues at most twice what the last one ran + 16, so frequent halts
+    // (sample_margin near 1, or logits out of the host's range every step) cost O(n) launches, not O(n^2).
+    unsigned long long chunk = n;
+    for (;;) {
+        rk::Ctrl &c = m->h_ctrl[0];
+        c = rk::Ctrl{0, tok, 0, done, 0};
+        CK(cudaMemcpyAsync(p.ctrl, &c, sizeof(rk::Ctrl), cudaMemcpyHostToDevice, m->stream));
+        const unsigned long long todo = std::min(n - done, chunk);
+        ep[0] = {m->epoch, m->tk};
+        for (unsigned long long i = 0; i < todo; ++i) {
+            if ((rc = launch_token(m, 1, !typ, nullptr, m->stream, true))) return rc;
+            ep[i + 1] = {m->epoch, m->tk};
+        }
+        CK(cudaMemcpyAsync(&c, p.ctrl, sizeof(rk::Ctrl), cudaMemcpyDeviceToHost, m->stream));
+        CK(cudaMemcpyAsync(h_t + done, d_t + done, todo * sizeof(unsigned long long), cudaMemcpyDeviceToHost, m->stream));
+        if (typ) CK(cudaMemcpyAsync(h_mg + done, d_mg + done, todo * sizeof(double), cudaMemcpyDeviceToHost, m->stream));
+        if (logits_out) CK(cudaMemcpyAsync(m->h_logits, dev_logits(m), V * sizeof(float), cudaMemcpyDeviceToHost, m->stream));
+        SYNC(m);
+        const unsigned long long ran = c.pos - done;
+        if (ran == 0 || ran > todo || (ran < todo && !c.halt))
+            return fail(8, "generate: the device ran %llu of %llu steps (halt %llu)", ran, todo, c.halt);
+        m->epoch = ep[ran].first;
+        m->tk = ep[ran].second;
+        done = c.pos;
+        const unsigned long long s = done - 1;
+        if (!c.halt) {
+            if (done == n) break;
+            tok = h_t[s]; // a bounded segment ran to its end
+            continue;
+        }
+        chunk = 2 * ran + 16;
+        if (typ && (!(h_mg[s] >= m->sample_margin) || h_mg[s] < 0.0)) {
+            // u too close to a boundary for the device's sums (or outside their range): the host's arithmetic decides
+            const float *lg = m->h_logits;
+            if (!logits_out) {
+                fallback_logits.resize(V);
+                CK(cudaMemcpy(fallback_logits.data(), dev_logits(m), V * sizeof(float), cudaMemcpyDeviceToHost));
+                lg = fallback_logits.data();
+            }
+            h_t[s] = (unsigned long long)typical_with_u(lg, temp, uniforms[s]);
+        }
+        tok = h_t[s];
+        if (done == n || is_stop(tok)) break;
+    }
+    memcpy(tokens_out, h_t, done * sizeof(unsigned long long));
+    *n_out = done;
+    if (logits_out && logits_out != m->h_logits) memcpy(logits_out, m->h_logits, V * sizeof(float));
+    return 0;
+}
+
 int rwkv_b200_decode_timed(rwkv_b200_model *m, const unsigned long long *tokens, unsigned long long n,
                            int teacher_forced, float *ms) {
     int rc = check_model(m);
@@ -867,6 +985,10 @@ int rwkv_b200_set_option(rwkv_b200_model *m, const char *key, const char *value)
         m->pf.disabled = v == 0;
     } else if (k == "prefill_graph") {
         m->pf.use_graph = v != 0;
+    } else if (k == "sample_margin") {
+        const double d = atof(value);
+        if (!(d >= 0.0 && d <= 1.0)) return fail(1, "sample_margin must be in [0, 1]");
+        m->sample_margin = d;
     } else if (k == "prefill_min") {
         if (v < 2) return fail(1, "prefill_min must be >= 2");
         m->pf.min_tokens = v;

@@ -84,7 +84,7 @@ struct Waiter {
     unsigned int spins;
 };
 __device__ __forceinline__ Waiter waiter_begin() { return Waiter{0ull, 0u}; }
-__device__ __noinline__ void wait_expired(const Params &p, unsigned int code, unsigned int layer, unsigned int kind,
+static __device__ __noinline__ void wait_expired(const Params &p, unsigned int code, unsigned int layer, unsigned int kind,
                                           unsigned int expect, unsigned int seen, unsigned long long aux) {
     Diag *d = p.diag;
     if (d != nullptr && atomicCAS(&d->code, 0u, code) == 0u) {

@@ -590,7 +590,7 @@ __device__ __forceinline__ void gather(const Params &p, const Smem &sm, const fl
 struct StatsOut {
     double mean, rstd;
 };
-__device__ __noinline__ StatsOut slice_stats(const Params &p, const double *xown, double *scal, long long *clkp, volatile uint32_t *quiet,
+static __device__ __noinline__ StatsOut slice_stats(const Params &p, const double *xown, double *scal, long long *clkp, volatile uint32_t *quiet,
                                              TaggedDouble *recs, int ne, uint32_t tag, unsigned int layer, int ctid, double c0,
                                              unsigned long long *trace) {
     struct {
@@ -760,7 +760,7 @@ __device__ __forceinline__ void publish_slice(const Smem &sm, TaggedDouble *recs
 // Sum over the G ranks of the partial result `part` of residual element j (a row-split GEMV): store it into
 // every peer's inbox, wait for the peers' parts, add in rank order (identical on every rank). Called by whole
 // warps (`valid` = this lane owns an element); the polling loop is warp-uniform.
-__device__ __noinline__ double peer_sum(const Params &p, unsigned int off_in, int j, double part, bool valid, uint32_t tag,
+static __device__ __noinline__ double peer_sum(const Params &p, unsigned int off_in, int j, double part, bool valid, uint32_t tag,
                                         unsigned int layer) {
     if (valid)
         for (int g = 0; g < p.G; ++g)
@@ -794,7 +794,7 @@ __device__ __noinline__ double peer_sum(const Params &p, unsigned int off_in, in
 }
 
 // sigmoid(ffn r) of residual element j, published by the owner of that channel (any rank). Whole warps.
-__device__ __noinline__ float peer_sr(const Params &p, int j, bool valid, uint32_t tag, unsigned int layer) {
+static __device__ __noinline__ float peer_sr(const Params &p, int j, bool valid, uint32_t tag, unsigned int layer) {
     const unsigned long long *srp = xch_at<unsigned long long>(p, p.rank, p.off_sr) + j;
     unsigned long long a = tag64(0u, tag);
     Waiter w = waiter_begin();
@@ -810,12 +810,223 @@ __device__ __noinline__ float peer_sr(const Params &p, int j, bool valid, uint32
     return __uint_as_float((uint32_t)a);
 }
 
-// CPL: 16-byte chunks per lane of an E-byte row segment; FULL: E == CPL * 512;
+// ---- the typical sampler over the head's logits (generate launches) ------------------------------------
+// The token is the one typical_with_u(logits, temp, u) returns (include/rwkv/sampler/typical.h): p_i ~ (exp(l_i) /
+// sum)^e with e = uint8(1 / temp), the first index whose sequential cumulative probability reaches u, cp_last
+// forced to 1. For e >= 1 the normalised distribution is softmax(e * l), so no CTA needs the global sum of exp(l)
+// before it can sum its powers: CTA b publishes {m_b = max of its logits, A_b = sum exp(l - m_b), B_b = sum exp(e
+// (l - m_b))} in ONE exchange (a second exchange for the global sum would add another all-to-all round trip to
+// every token) and every reader rescales to the global maximum M, so nothing overflows whatever e is. Every CTA
+// builds the prefix P over the CTAs from the same words with the same fixed-shape scan, so all agree on every
+// boundary and exactly one finds u in its interval (P_b, P_b+1] (CTA 0's closed at 0, the last one open to the
+// top: cp_last = 1 and u < 1). That CTA scans its own rows (block scan of the logits recomputed from the integer row
+// totals in shared memory) and finishes the step: token and margin into the run's arrays at ctrl->pos, the token
+// into ctrl->next, and the halt flag when the margin is below margin_min or the token is a stop id. The device sums
+// differ from the host's sequential ones by ~1e-13, hence the margin; where the host's own arithmetic leaves the
+// range of doubles (its sum of exp(l) over the vocabulary overflows once max l > 709.78 - ln(V); (exp(l) / sum)^e
+// underflows for a large e: A_b gives the host's sum), and where rounding left u above the claiming CTA's own
+// running sum, the margin is reported as -1: the step always halts and the host decides with its own arithmetic.
+__device__ __forceinline__ bool is_stop(const Params &p, unsigned long long t) {
+    bool stop = false;
+#pragma unroll
+    for (int k = 0; k < kMaxStop; ++k) stop = stop || (k < p.n_stop && p.stop[k] == t);
+    return stop;
+}
+__device__ __forceinline__ void sample_head(const Params &p, const Smem &sm, int v0, int nv, int ctid) {
+    // the step index: written by this step's finishing CTA only after it has this CTA's record (published below)
+    const unsigned long long pos = p.ctrl->pos;
+    const int lane = ctid & 31, w = ctid >> 5, nb = (int)gridDim.x, b = (int)blockIdx.x;
+    const int e = p.exponent;
+    const double de = (double)e;
+    auto logit = [&](int i) { return (float)(sm.scal[0] * (double)sm.res64[i] + sm.scal[3]); };
+    auto power = [&](double d) { return e == 0 ? 1.0 : e == 1 ? exp(d) : exp(de * d); }; // exp(l - m)^e
+    double *sh = sm.osum;                                        // [kWarps * 3] scratch
+    uint32_t *wm = sm.wmax;                                      // [kWarps]
+    float mx = -INFINITY;
+    for (int i = ctid; i < nv; i += kConsumers) mx = fmaxf(mx, logit(i));
+    __syncwarp();
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+    if (lane == 0) sh[w] = (double)mx;
+    tok_sync();
+    double m = sh[0];
+    for (int k = 1; k < kWarps; ++k) m = fmax(m, sh[k]);
+    if (!(m > -INFINITY)) m = 0.0; // no finite logit: the sums below are NaN or 0 and the host decides
+    tok_sync();
+    double a = 0.0, bs = 0.0;
+    for (int i = ctid; i < nv; i += kConsumers) {
+        const double d = (double)logit(i) - m;
+        a += exp(d);
+        bs += power(d);
+    }
+    a = warp_sum(a);
+    bs = warp_sum(bs);
+    if (lane == 0) {
+        sh[w * 3 + 0] = a;
+        sh[w * 3 + 1] = bs;
+    }
+    tok_sync();
+    if (w == 0) {
+        double A = 0.0, B = 0.0;
+        for (int k = 0; k < kWarps; ++k) { // warps in order: the same bits in every lane
+            A += sh[k * 3 + 0];
+            B += sh[k * 3 + 1];
+        }
+        TaggedDouble *const recs = xch_at<TaggedDouble>(p, p.rank, p.off_smp);
+        if (lane < kRep) {
+            st_tagged_double(&recs[((size_t)lane * 3 + 0) * nb + b], m, p.tk, false);
+            st_tagged_double(&recs[((size_t)lane * 3 + 1) * nb + b], A, p.tk, false);
+            st_tagged_double(&recs[((size_t)lane * 3 + 2) * nb + b], B, p.tk, false);
+        }
+        // lane l holds records l*kPer .. l*kPer + kPer - 1 (contiguous: the prefix is a lane-local sum + one warp scan)
+        constexpr int kPer = (kMaxGrid + 31) / 32;
+        const TaggedDouble *const rd = recs + (size_t)(b % kRep) * 3 * nb;
+        const unsigned long long none = tag64(0u, p.tk);
+        unsigned long long ra[kPer][3], rb[kPer][3];
+#pragma unroll
+        for (int i = 0; i < kPer; ++i) {
+            const int r = lane * kPer + i;
+#pragma unroll
+            for (int k = 0; k < 3; ++k) {
+                ra[i][k] = rb[i][k] = none;
+                if (r < nb) ld_pair(&rd[(size_t)k * nb + r], ra[i][k], rb[i][k], false);
+            }
+        }
+        Waiter wt = waiter_begin();
+        for (;;) {
+            bool bad = false;
+#pragma unroll
+            for (int i = 0; i < kPer; ++i)
+#pragma unroll
+                for (int k = 0; k < 3; ++k)
+                    if (!tags_ok(ra[i][k], rb[i][k], p.tk)) {
+                        ld_pair(&rd[(size_t)k * nb + lane * kPer + i], ra[i][k], rb[i][k], false);
+                        bad = true;
+                    }
+            if (!__any_sync(0xffffffffu, bad)) break; // warp-uniform exit (see slice_stats)
+            if (waiter_tick(p, wt)) wait_expired(p, kDiagSample, (unsigned int)p.L_run, 0, p.tk, (unsigned int)(ra[0][0] >> 32), (unsigned long long)lane);
+        }
+        double M = -INFINITY;
+#pragma unroll
+        for (int i = 0; i < kPer; ++i)
+            if (lane * kPer + i < nb) M = fmax(M, pair_to_double(ra[i][0], rb[i][0]));
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) M = fmax(M, __shfl_xor_sync(0xffffffffu, M, o));
+        double P[kPer], run = 0.0, asum = 0.0;
+#pragma unroll
+        for (int i = 0; i < kPer; ++i) {
+            double wgt = 0.0;
+            if (lane * kPer + i < nb) {
+                const double mb = pair_to_double(ra[i][0], rb[i][0]);
+                const double Bb = pair_to_double(ra[i][2], rb[i][2]);
+                wgt = e == 0 ? Bb : exp(de * (mb - M)) * Bb;
+                asum += exp(mb - M) * pair_to_double(ra[i][1], rb[i][1]);
+            }
+            P[i] = run;
+            run += wgt;
+        }
+        double incl = run;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const double y = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += y;
+        }
+        double excl = __shfl_up_sync(0xffffffffu, incl, 1);
+        if (lane == 0) excl = 0.0;
+        const double S = __shfl_sync(0xffffffffu, incl, 31);
+        asum = warp_sum(asum);
+        double lo = 0.0, hi = 0.0;
+#pragma unroll
+        for (int i = 0; i < kPer; ++i) {
+            const double Pr = excl + P[i]; // the same formula for every record in every CTA
+            if (lane * kPer + i == b) lo = Pr;
+            if (lane * kPer + i == b + 1) hi = Pr;
+        }
+        lo = __shfl_sync(0xffffffffu, lo, b / kPer) / S;
+        hi = b + 1 < nb ? __shfl_sync(0xffffffffu, hi, (b + 1) / kPer) / S : 2.0;
+        const double u = p.uniforms[pos];
+        const bool claim = (b == 0 || lo < u) && !(hi < u);
+        bool ok = S > 0.0 && S < INFINITY;
+        // host: sum of exp(l) <= V exp(M) must stay finite (709.78 = ln of the largest double), exp(l) normal
+        if (e >= 1) ok = ok && M <= 709.0 - log((double)kVocab) && M >= -600.0;
+        if (e >= 2) ok = ok && log(S) - de * log(asum) > -650.0;
+        if (lane == 0) {
+            sh[0] = claim ? 1.0 : 0.0;
+            sh[1] = lo;
+            sh[2] = (e == 0 ? 1.0 : exp(de * (m - M))) / S; // own rows: p_i = exp(l_i - m)^e * f
+            sh[3] = u;
+            sh[4] = ok ? 1.0 : 0.0;
+        }
+    }
+    tok_sync();
+    if (sh[0] == 0.0) return; // block-uniform
+    const double f = sh[2], u = sh[3];
+    const bool ok = sh[4] != 0.0;
+    double carry = sh[1];
+    tok_sync(); // sh is reused below
+    int found = -1;
+    double fmargin = 0.0;
+    for (int c0 = 0; c0 < nv; c0 += kConsumers) {
+        const int i = c0 + ctid;
+        const bool valid = i < nv;
+        const double pi = valid ? power((double)logit(i) - m) * f : 0.0;
+        double x = pi;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const double y = __shfl_up_sync(0xffffffffu, x, o);
+            if (lane >= o) x += y;
+        }
+        double xex = __shfl_up_sync(0xffffffffu, x, 1);
+        if (lane == 0) xex = 0.0;
+        if (lane == 31) sh[w] = x;
+        tok_sync();
+        double woff = 0.0, tot = 0.0;
+        for (int k = 0; k < kWarps; ++k) {
+            if (k < w) woff += sh[k];
+            tot += sh[k];
+        }
+        const double c = carry + (woff + x), prev = carry + (woff + xex);
+        const bool last = b == nb - 1 && i == nv - 1;
+        const uint32_t cand = valid && (last || !(c < u)) ? (uint32_t)i : 0xffffffffu;
+        const uint32_t wmin = __reduce_min_sync(0xffffffffu, cand);
+        if (lane == 0) wm[w] = wmin;
+        tok_sync();
+        uint32_t first = wm[0];
+        for (int k = 1; k < kWarps; ++k) first = min(first, wm[k]);
+        if (first != 0xffffffffu) {
+            found = (int)first;
+            if ((uint32_t)i == first) fmargin = last ? u - prev : fmin(u - prev, c - u);
+            break; // block-uniform
+        }
+        carry = carry + tot;
+        tok_sync();
+    }
+    // rounding left u above this CTA's own running sum (found < 0): no trusted token, the host decides
+    const bool writer = found >= 0 ? ctid == found - (found / kConsumers) * kConsumers : ctid == 0;
+    if (writer) {
+        const unsigned long long t = (unsigned long long)(p.vbase + v0 + (found >= 0 ? found : nv - 1));
+        const double margin = !ok || found < 0 ? -1.0 : fmargin;
+        p.gen_tokens[pos] = t;
+        p.gen_margins[pos] = margin;
+        p.ctrl->next = t;
+        p.ctrl->pos = pos + 1;
+        if (is_stop(p, t) || !(margin >= p.margin_min)) p.ctrl->halt = 1;
+    }
+}
+
+// CPL: 16-byte chunks per lane of an E-byte row segment (the values instantiated: RK_CPLS); FULL: E == CPL * 512;
 // TRACE: with the %globaltimer stamps of tools/trace_token.py (set_option("trace", 1)).
-template <int CPL, bool FULL, bool TRACE>
+// GEN: a step of rwkv_b200_generate - halted launches exit at entry, the head finishes with the arg-max (p.greedy)
+// or the typical sampler and records the step (a separate instantiation: the other launches keep their code).
+#define RK_CPLS(X) X(2) X(4) X(6) X(8) X(10)
+template <int CPL, bool FULL, bool TRACE, bool GEN = false>
 __global__ void __launch_bounds__(kThreads, 1) k_token(const __grid_constant__ Params p) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     const Smem sm = carve(smem_raw, p);
+    // generate: the halt flag was written by the previous launch; every thread reads it before the barrier below, so
+    // the CTA that finishes this step (after every CTA has published) cannot race it
+    bool halted = false;
+    if constexpr (GEN) halted = p.ctrl->halt != 0;
     if (threadIdx.x == 0) {
         for (int i = 0; i < p.stages; ++i) {
             mbar_init(smem_u32(&sm.full[i]), 1);
@@ -826,6 +1037,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_token(const __grid_constant__ P
         mbar_fence_init();
     }
     __syncthreads();
+    if constexpr (GEN) {
+        if (halted) return; // uniform over the grid: no exchange, no state write, epochs untouched
+    }
     if (p.cluster > 1) cluster_sync_all(); // the peers' barriers exist before anybody arrives on them
     const int E = p.E, Er = p.Er;
     const int nb = (int)gridDim.x;
@@ -1283,6 +1497,13 @@ __global__ void __launch_bounds__(kThreads, 1) k_token(const __grid_constant__ P
                                 i2 = bi[w2];
                             }
                         p.ctrl->next = (unsigned long long)(i2 == 0x7fffffff ? 0 : i2);
+                        if constexpr (GEN) {
+                            const unsigned long long t = (unsigned long long)(i2 == 0x7fffffff ? 0 : i2);
+                            const unsigned long long pos = p.ctrl->pos; // this thread is its only writer
+                            p.gen_tokens[pos] = t;
+                            p.ctrl->pos = pos + 1;
+                            if (is_stop(p, t)) p.ctrl->halt = 1;
+                        }
                     }
                 }
             }
@@ -1319,6 +1540,13 @@ __global__ void __launch_bounds__(kThreads, 1) k_token(const __grid_constant__ P
             }
             __threadfence_system();
         }
+    }
+    // the sampler runs after the phase loop (the logits' row totals stay in shared memory) and is inlined: compiled as
+    // a called function it gave the kernel local-memory traffic on the layer path (192-byte stack instead of 64) and
+    // generate ran 11.6 % (1.5B) and 6.5 % (7B) slower per token than decode_timed; inlined, both run at the same
+    // speed (profiles/r03_generate_breakdown.txt)
+    if constexpr (GEN) {
+        if (!p.greedy) sample_head(p, sm, sl.v0, sl.nv, ctid);
     }
     if (blockIdx.x == 0 && ctid == 0 && p.feed_mode == 2) p.ctrl->pos = p.ctrl->pos + 1;
     if ((p.dbg & 4) && p.trace != nullptr && ctid == 0)

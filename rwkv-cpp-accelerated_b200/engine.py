@@ -10,6 +10,7 @@ import numpy as np
 
 VOCAB = 50277
 MODE_PARRALEL, MODE_GPT = 0, 1
+GEN_GREEDY, GEN_TYPICAL = 0, 1
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
@@ -56,6 +57,7 @@ def load_library():
         "rwkv_b200_forward_greedy": (i32, [vp, ull, pull, pflt]),
         "rwkv_b200_logits_host": (pflt, [vp]),
         "rwkv_b200_sample_typical": (i32, [vp, c.c_float, c.c_double, pull, pdbl]),
+        "rwkv_b200_generate": (i32, [vp, ull, ull, i32, c.c_float, pdbl, pull, i32, pull, pull, pflt]),
         "rwkv_b200_debug_read": (c.c_longlong, [vp, cp, vp, c.c_size_t]),
         "rwkv_b200_decode_timed": (i32, [vp, pull, ull, i32, pflt]),
         "rwkv_b200_kernel_count": (i32, []),
@@ -146,6 +148,23 @@ class Engine:
         tok, margin = ctypes.c_ulonglong(), ctypes.c_double()
         self._ck(self.lib.rwkv_b200_sample_typical(self.h, temp, u, ctypes.byref(tok), ctypes.byref(margin)), "sample_typical")
         return int(tok.value), float(margin.value)
+
+    def generate(self, first, n, how=GEN_TYPICAL, temp=0.9, uniforms=None, stop=(), want_logits=True):
+        """rwkv_b200_generate: n steps of forward + pick (GEN_GREEDY: arg-max; GEN_TYPICAL: the typical sampler with
+        uniforms[i] at step i) from token `first` on the device. Returns (tokens t1..tk, the last step's logits or None);
+        k < n only when tk is in `stop`."""
+        out = np.empty(max(int(n), 1), np.uint64)
+        k = ctypes.c_ulonglong()
+        u = None if uniforms is None else np.ascontiguousarray(uniforms, dtype=np.float64)
+        if u is not None and u.size < n:
+            raise EngineError("generate: %d uniforms for %d steps" % (u.size, n))
+        st = np.ascontiguousarray(np.asarray(list(stop), dtype=np.uint64)) if len(stop) else None
+        lg = np.empty(VOCAB, np.float32) if want_logits else None
+        self._ck(self.lib.rwkv_b200_generate(self.h, int(first), int(n), int(how), float(temp), _ptr(u, ctypes.c_double),
+                                             _ptr(st, ctypes.c_ulonglong), 0 if st is None else len(st),
+                                             _ptr(out, ctypes.c_ulonglong), ctypes.byref(k), _ptr(lg, ctypes.c_float)),
+                 "generate")
+        return [int(t) for t in out[:k.value]], lg
 
     def forward_greedy(self, token, want_logits=False):
         nxt = ctypes.c_ulonglong()
